@@ -20,6 +20,7 @@ be built here: Eigen/PCL/yaml-cpp absent and its "Ours" stage is a stub) on the 
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -77,6 +78,7 @@ class ClockSampler:
                                          stdout=open(self.path, "w"), stderr=subprocess.DEVNULL)
         except Exception:
             self.proc = None
+        atexit.register(self.stop)                         # a run that fails mid-way must not leave nvidia-smi polling
 
     def stop(self):
         out = {"sm_mhz": None, "sm_max_mhz": None, "reasons": [], "samples": 0}
@@ -88,6 +90,7 @@ class ClockSampler:
             self.proc.wait(timeout=5)
         except Exception:
             self.proc.kill()
+        self.proc = None
         sm, mx, reasons = [], [], set()
         try:
             for ln in open(self.path):
@@ -118,6 +121,27 @@ def c2_params(default_params):
     return default_params(search_radius=1.0, max_iterations=C2_ITERS, fixed_iterations=1, kappa_target=10.0,
                           cond_thresh=10.0, use_weight_derivative=0, detection="SCHUR_CONDITION_NUMBER",
                           handling="PRECONDITIONED_CG")
+
+
+def result_arrays(prefix, r):
+    """What one ICP call handed back (an IcpResult) as arrays named <prefix>_<what>: the pose, iteration count and
+    flags, and every per-iteration log field stacked over the iterations.  The log's wall-clock iter_time_ms and the
+    reserved padding are left out: they are not results and would differ between identical runs."""
+    from dcreg_b200.api import Analysis, IterLog
+    out = {f"{prefix}_pose": r.T, f"{prefix}_iterations": r.iterations, f"{prefix}_converged": r.converged,
+           f"{prefix}_status": r.status}
+    for struct, part in ((IterLog, lambda L: L), (Analysis, lambda L: L.analysis)):
+        for name, _ in struct._fields_:
+            if r.logs and name not in ("analysis", "iter_time_ms", "reserved1"):
+                out[f"{prefix}_log_{name}"] = [np.array(getattr(part(L), name)) for L in r.logs]
+    return out
+
+
+def write_outputs(directory, arrays):
+    """--dump-outputs: DIR/<name>.npy, float64, one file per array."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -309,7 +333,9 @@ def run_reference(args, rank, world):
         return
     arm = CpuArm(seed=42)
     arm.calibrate()
-    times, _ = arm.steps(args.steps, args.warmup)
+    times, T = arm.steps(args.steps, args.warmup)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"c2_pose": T})
     cpu = arm.describe(times)
     cpu["reference_faithful_8_threads"] = arm.faithful()
     value = cpu["value"]
@@ -384,6 +410,7 @@ def run_ours(args, rank, local_rank, world):
     e1.synchronize()
     res = ctx.icp_fetch()
     assert res.iterations == C2_ITERS
+    outputs = result_arrays("c2", res)
     barrier()
     dev_ms = max_over_ranks(e0.elapsed_time(e1))
     launches = ctx.launch_count - l0
@@ -410,6 +437,7 @@ def run_ours(args, rank, local_rank, world):
     e3.record(stream)
     e3.synchronize()
     wall = time.perf_counter() - w0
+    outputs.update(result_arrays("e2e", res))
     barrier()
     e2e_ms = max_over_ranks(max(e2.elapsed_time(e3), wall * 1e3))
     clocks = sampler.stop() if rank == 0 else None
@@ -469,6 +497,7 @@ def run_ours(args, rank, local_rank, world):
     f1.synchronize()
     barrier()
     c4_ms = max_over_ranks(f0.elapsed_time(f1)) / c4_runs
+    outputs.update(result_arrays("c4", res4))
     comm_mode = ctx.comm_mode
     sharded_ok, sharded_dT = None, None
     ctx2 = Context(local_rank)                                               # plain context: no communicator
@@ -522,6 +551,8 @@ def run_ours(args, rank, local_rank, world):
     w5 = time.perf_counter() - w5
     barrier()
     c5_ms = max_over_ranks(max(g0.elapsed_time(g1), w5 * 1e3))
+    per_trial = [result_arrays("c5", t) for t in trials]
+    outputs.update({k: [p[k] for p in per_trial] for k in per_trial[0]})
     n_conv = torch.tensor([float(sum(t.converged for t in trials)), float(sum(t.iterations for t in trials))],
                           dtype=torch.float64, device=dev)
     if world > 1:
@@ -563,6 +594,8 @@ def run_ours(args, rank, local_rank, world):
             cpu = host["cpu_baseline"]
             c5["cpu_port"] = host["c5_cpu"]
 
+    if rank == 0 and args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
     if rank == 0:
         line = {
             "metric": "icp_iterations_per_s", "value": value, "unit": "ICP iterations/s", "n_gpus": world,
@@ -612,9 +645,15 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the run, write what the timed calls returned in their last step as DIR/<name>.npy "
+                         "(float64; rank 0): c2_* the flagship step, e2e_* the host-buffer step, c4_* the corridor "
+                         "registration, c5_* the Monte-Carlo trials; the reference arm writes c2_pose")
     ap.add_argument("--cpu-worker", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--cpu-trials", action="store_true", help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
     if args.cpu_worker:
         pin_openmp_env(host_cpu_budget()[0])

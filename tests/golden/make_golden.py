@@ -1,10 +1,11 @@
 #!/usr/bin/env python
 """Extract the reference's shipped golden vectors into tests/golden/golden.json.
 
-Run HERE (needs /root/reference, which does not exist on the GPU box):
-    python tests/golden/make_golden.py
+Needs a checkout of the reference project (JokerJohn/DCReg with its shipped results); the tests only read the
+golden.json this writes:
+    python tests/golden/make_golden.py <reference checkout>
 
-Sources (SURVEY.md §8c), all relative to /root/reference:
+Sources (SURVEY.md §8c), all relative to the reference checkout:
   G1  DCReg/dataset/icp_results/            released code, init t=(0.01,0.01,0.01), WD off
   G2  results/simulation/table3_fig9_fig10/ full code incl. "Ours", init (0.2,0.8,0.5 m;
                                             0.1,0.1,2 deg), weight derivative ON
@@ -16,8 +17,8 @@ import csv
 import json
 import os
 import re
+import sys
 
-REF = "/root/reference"
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 DX = ["dx_wx", "dx_wy", "dx_wz", "dx_x", "dx_y", "dx_z"]
@@ -85,10 +86,10 @@ def first_iter_blocks(path):
     return out
 
 
-def main():
+def main(ref):
     g = {"_source": "JokerJohn/DCReg @ 0519bdb shipped result dumps; see make_golden.py"}
     so3 = {"Ours", "ME-SR", "ME-TSVD", "ME-TReg", "FCN-SR"}
-    g1 = os.path.join(REF, "DCReg/dataset/icp_results")
+    g1 = os.path.join(ref, "DCReg/dataset/icp_results")
     g["G1"] = {
         "setup": {"init_xyz": [0.01, 0.01, 0.01], "init_rpy_deg": [0, 0, 0], "use_weight_derivative": False,
                   "search_radius": 1.0, "conv_rot": 1e-4, "conv_trans": 1e-3, "std_reg_gamma": 100.0,
@@ -96,7 +97,7 @@ def main():
         "iterations": rows_of(os.path.join(g1, "iteration_details_with_dx.csv"), so3),
         "first_iter": first_iter_blocks(os.path.join(g1, "degeneracy_analysis_first_iter.txt")),
     }
-    g2 = os.path.join(REF, "results/simulation/table3_fig9_fig10")
+    g2 = os.path.join(ref, "results/simulation/table3_fig9_fig10")
     g["G2"] = {
         "setup": {"init_xyz": [0.2, 0.8, 0.5], "init_rpy_deg": [0.1, 0.1, 2.0], "use_weight_derivative": True,
                   "search_radius": 1.0, "conv_rot": 1e-5, "conv_trans": 1e-3, "std_reg_gamma": 100.0,
@@ -106,7 +107,7 @@ def main():
         "schur_lambda_rot": [422.505477, 1447.735216, 2999.323349],
         "schur_lambda_trans": [0.629416, 5.601848, 16.871859],
     }
-    g3 = os.path.join(REF, "results/simulation/fig8_5000iters")
+    g3 = os.path.join(ref, "results/simulation/fig8_5000iters")
     keep = set(range(0, 40)) | {99, 999, 4999}
     g["G3"] = {
         "setup": dict(g["G2"]["setup"], conv_rot=1e-14, conv_trans=1e-12, max_iterations=5000),
@@ -118,4 +119,6 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    main(sys.argv[1])

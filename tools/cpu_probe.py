@@ -1,5 +1,6 @@
 import sys, os, time
-sys.path.insert(0,'/root/repo/oracle'); sys.path.insert(0,'/root/repo')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, 'oracle')); sys.path.insert(0, ROOT)
 if os.environ.get('WITH_TORCH'): import torch
 import dcreg_oracle_c as oc
 from dcreg_b200.scenes import make_cylinder, g2_initial_pose
