@@ -87,7 +87,7 @@ EXPORTS = [
     "dcreg_stream", "dcreg_set_source", "dcreg_set_target", "dcreg_find_planes",
     "dcreg_reduce_normal_equations", "dcreg_reduce_normal_equations_f64plane",
     "dcreg_reduce_normal_equations_host", "dcreg_analyze_and_solve", "dcreg_solve_pcg", "dcreg_icp_run",
-    "dcreg_icp_run_batch", "dcreg_icp_enqueue", "dcreg_icp_fetch", "dcreg_icp_run_host_planes", "dcreg_comm_mode", "dcreg_last_covariance", "dcreg_point_to_point_metrics", "dcreg_comm_unique_id", "dcreg_comm_init",
+    "dcreg_icp_run_batch", "dcreg_icp_run_scans", "dcreg_icp_enqueue", "dcreg_icp_fetch", "dcreg_icp_run_host_planes", "dcreg_comm_mode", "dcreg_last_covariance", "dcreg_last_covariances", "dcreg_point_to_point_metrics", "dcreg_comm_unique_id", "dcreg_comm_init",
     "dcreg_comm_destroy", "dcreg_set_global_source_count", "dcreg_launch_count", "dcreg_device_source",
     "dcreg_device_planes_f64", "dcreg_device_planes_f32", "dcreg_freeze_planes_f32", "dcreg_time_reduce", "dcreg_time_iteration", "dcreg_iteration_counters", "dcreg_iteration_timeline",
 ]
@@ -122,12 +122,15 @@ def load_library():
                                   C.POINTER(ci)]
     lib.dcreg_icp_run_batch.argtypes = [vp, C.POINTER(IcpParams), ci, dp, dp, C.POINTER(ci), C.POINTER(ci), C.POINTER(ci),
                                         C.POINTER(IterLog), ci]
+    lib.dcreg_icp_run_scans.argtypes = [vp, C.POINTER(IcpParams), ci, C.POINTER(C.c_float), ci, C.POINTER(i64), dp, dp,
+                                        C.POINTER(ci), C.POINTER(ci), C.POINTER(ci), C.POINTER(IterLog), ci]
     lib.dcreg_comm_mode.argtypes = [vp]
     lib.dcreg_icp_enqueue.argtypes = [vp, C.POINTER(IcpParams), dp]
     lib.dcreg_icp_fetch.argtypes = [vp, dp, C.POINTER(ci), C.POINTER(ci)]
     lib.dcreg_icp_run_host_planes.argtypes = [vp, C.POINTER(IcpParams), dp, PLANE_CALLBACK, vp, dp,
                                               C.POINTER(IterLog), ci, C.POINTER(ci), C.POINTER(ci)]
     lib.dcreg_last_covariance.argtypes = [vp, dp]
+    lib.dcreg_last_covariances.argtypes = [vp, ci, dp]
     lib.dcreg_point_to_point_metrics.argtypes = [vp, dp, C.c_double, dp]
     lib.dcreg_comm_unique_id.argtypes = [vp, C.POINTER(C.c_uint8)]
     lib.dcreg_comm_init.argtypes = [vp, C.POINTER(C.c_uint8), ci, ci]
@@ -179,6 +182,30 @@ def _as_points(xyz):
 def pose_Rt(T):
     T = np.asarray(T, dtype=np.float64)
     return np.ascontiguousarray(np.concatenate([T[:3, :3].reshape(-1), T[:3, 3]]))
+
+
+def pack_scans(scans):
+    """A list of (N_i, >=3) point arrays -> (xyz (sum N_i, 3) float32, offsets (n + 1,) int64): scan i is
+    xyz[offsets[i]:offsets[i + 1]], the layout dcreg_icp_run_scans takes.  Columns past the third are dropped."""
+    parts = [_as_points(s)[:, :3] for s in scans]
+    if not parts:
+        raise ValueError("no scans")
+    offsets = np.zeros(len(parts) + 1, dtype=np.int64)
+    offsets[1:] = np.cumsum([p.shape[0] for p in parts])
+    return np.ascontiguousarray(np.concatenate(parts, axis=0), dtype=np.float32), offsets
+
+
+def _batch_results(B, T_out, n_it, conv, st, logs, cap):
+    out = []
+    for b in range(B):
+        recs = []
+        if logs is not None:
+            nrec = min(n_it[b], cap)
+            if st[b] == NONFINITE_UPDATE and n_it[b] < cap:
+                nrec = n_it[b] + 1
+            recs = [logs[b * cap + i] for i in range(nrec)]
+        out.append(IcpResult(int(st[b]), bool(conv[b]), int(n_it[b]), T_out[b], recs))
+    return out
 
 
 class IcpResult:
@@ -364,16 +391,25 @@ class Context:
         logs = (IterLog * max(cap * B, 1))() if want_log else None
         self._check(self.lib.dcreg_icp_run_batch(self._h, C.byref(params), B, _dptr(T_init), _dptr(T_out), n_it, conv, st,
                                                  logs, cap))
-        out = []
-        for b in range(B):
-            recs = []
-            if want_log:
-                nrec = min(n_it[b], cap)
-                if st[b] == NONFINITE_UPDATE and n_it[b] < cap:
-                    nrec = n_it[b] + 1
-                recs = [logs[b * cap + i] for i in range(nrec)]
-            out.append(IcpResult(int(st[b]), bool(conv[b]), int(n_it[b]), T_out[b], recs))
-        return out
+        return _batch_results(B, T_out, n_it, conv, st, logs, cap)
+
+    def icp_run_scans(self, params: IcpParams, scans, T_init, want_log: bool = False):
+        """Many different scans against the context's target, side by side: scans = list of (N_i, >=3) arrays,
+        T_init (n, 4, 4), one initial pose per scan.  Returns a list of IcpResult, one per scan (logs only when
+        want_log).  The context's source (set_source) is left as it was."""
+        xyz, offsets = pack_scans(scans)
+        B = offsets.size - 1
+        T_init = np.ascontiguousarray(T_init, dtype=np.float64).reshape(-1, 4, 4)
+        if T_init.shape[0] != B:
+            raise ValueError(f"{B} scans but {T_init.shape[0]} initial poses")
+        T_out = np.empty((B, 4, 4))
+        n_it = (C.c_int * B)(); conv = (C.c_int * B)(); st = (C.c_int * B)()
+        cap = int(params.max_iterations) if want_log else 0
+        logs = (IterLog * max(cap * B, 1))() if want_log else None
+        self._check(self.lib.dcreg_icp_run_scans(self._h, C.byref(params), B, xyz.ctypes.data_as(C.POINTER(C.c_float)),
+                                                 xyz.shape[1], offsets.ctypes.data_as(C.POINTER(C.c_int64)),
+                                                 _dptr(T_init), _dptr(T_out), n_it, conv, st, logs, cap))
+        return _batch_results(B, T_out, n_it, conv, st, logs, cap)
 
     def icp_run_host_planes(self, params: IcpParams, T_init, plane_fn, want_log: bool = True) -> IcpResult:
         """Same loop with caller-supplied correspondences: plane_fn(T 4x4) -> (planes (N,4) f64, n_corr_pt)."""
@@ -409,6 +445,13 @@ class Context:
     def last_covariance(self):
         cov = np.empty((6, 6))
         self._check(self.lib.dcreg_last_covariance(self._h, _dptr(cov)))
+        return cov
+
+    def last_covariances(self, n: int):
+        """Covariance of each of the first n trials of the last run (icp_run: 1; icp_run_batch / icp_run_scans: their
+        count), shape (n, 6, 6)."""
+        cov = np.empty((int(n), 6, 6))
+        self._check(self.lib.dcreg_last_covariances(self._h, int(n), _dptr(cov)))
         return cov
 
     def point_to_point_metrics(self, T, error_threshold: float):

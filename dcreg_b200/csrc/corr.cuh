@@ -208,12 +208,8 @@ __global__ void grid_rank_cells_kernel(const float4* __restrict__ in, int n, con
     if (pos_of) pos_of[me] = s + rank;
 }
 
-// cell of a (transformed) source point for the spatial sort of the source cloud, clamped into the target box
-__global__ void source_cell_kernel(const float4* __restrict__ src, int n, Grid g, const double* __restrict__ T,
-                                   int* __restrict__ pt_cell, int* __restrict__ counts) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const float4 p = src[i];
+// dense cell of T*p (T: row-major 4x4, first three rows read), clamped into the target box
+__device__ __forceinline__ int source_cell(const float4 p, const Grid& g, const double* __restrict__ T) {
     const double px = p.x, py = p.y, pz = p.z;
     const float qx = (float)(T[0] * px + T[1] * py + T[2] * pz + T[3]);
     const float qy = (float)(T[4] * px + T[5] * py + T[6] * pz + T[7]);
@@ -221,9 +217,46 @@ __global__ void source_cell_kernel(const float4* __restrict__ src, int n, Grid g
     const int cx = min(max(cell_coord(qx, g.inv_cell) - g.ox, 0), g.nx - 1);
     const int cy = min(max(cell_coord(qy, g.inv_cell) - g.oy, 0), g.ny - 1);
     const int cz = min(max(cell_coord(qz, g.inv_cell) - g.oz, 0), g.nz - 1);
-    const int c = (cz * g.ny + cy) * g.nx + cx;
+    return (cz * g.ny + cy) * g.nx + cx;
+}
+
+// cell of a (transformed) source point for the spatial sort of the source cloud
+__global__ void source_cell_kernel(const float4* __restrict__ src, int n, Grid g, const double* __restrict__ T,
+                                   int* __restrict__ pt_cell, int* __restrict__ counts) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int c = source_cell(src[i], g, T);
     pt_cell[i] = c;
     atomicAdd(&counts[c], 1);
+}
+
+// Scan s of a scan set = slots [off[s], off[s+1]) (off strictly increasing, off[0] = 0): the s with off[s] <= i < off[s+1].
+__device__ __forceinline__ int scan_of(const long long* __restrict__ off, int n_scans, long long i) {
+    int lo = 0, hi = n_scans - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (__ldg(&off[mid]) <= i) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// Sort keys of a scan set: (scan << 32) | target cell of T_s * p with T = [n_scans][16]; value = slot.  A stable radix sort
+// on these keys keeps every scan contiguous and, inside a cell, the input order - for one scan exactly the order of the
+// counting sort above (source_cell_kernel + grid_scatter_kernel + grid_rank_cells_kernel).
+__global__ void scan_cell_keys_kernel(const float4* __restrict__ src, int n, const long long* __restrict__ off, int n_scans,
+                                      Grid g, const double* __restrict__ T, unsigned long long* __restrict__ keys,
+                                      int* __restrict__ slots) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int s = scan_of(off, n_scans, i);
+    keys[i] = ((unsigned long long)s << 32) | (unsigned)source_cell(src[i], g, T + (size_t)s * 16);
+    slots[i] = i;
+}
+
+// sorted[j] = src[slot[j]] (w keeps the point's slot in the unsorted buffer)
+__global__ void gather_points_kernel(const float4* __restrict__ src, int n, const int* __restrict__ slot, float4* __restrict__ out) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j < n) out[j] = src[slot[j]];
 }
 
 // ---- query -----------------------------------------------------------------------------------

@@ -2,6 +2,7 @@
 
 C2  make_cylinder : the shipped cylinder's geometry (wall R = 40 m, z in [0, 20] + floor disc z = 0) at any size
 C3  make_parking  : ground-dominated local map + sparse verticals, LiDAR-like frame (stand-in, pair not shipped)
+    make_parking_sequence : a sequence of ragged frames along a path over the same map (scan-to-map batches)
 C4  make_corridor : two parallel walls + floor + ceiling, rank-deficient along x
 C5  trial_poses   : seeded perturbations t ~ U[-1, 1]^3 m, rpy ~ U[-3, 3]^3 deg for the Monte-Carlo (SURVEY.md §8d)
     load_pcd_xyz  : PCD v0.7 `DATA binary` with float32 fields (the shipped clouds, SURVEY.md Appendix B.3)
@@ -83,6 +84,35 @@ def make_parking(n_map=500_000, n_scan=6_000, seed=43, extent=60.0, max_range=30
     pick = rng.choice(cand, size=min(n_scan, cand.size), replace=False)
     scan = (tgt[pick].astype(np.float64) + rng.normal(0, 0.005, (pick.size, 3))).astype(np.float32)
     return np.ascontiguousarray(scan), np.ascontiguousarray(tgt)
+
+
+def make_parking_sequence(n_scans, seed=46, n_map=500_000, path_radius=20.0, max_range=30.0, min_points=3_000,
+                          max_points=8_000, noise=0.005):
+    """A recorded sequence over make_parking's map: returns (scans, map, T_gt, T_init).
+
+    The vehicle drives one lap of a circle of radius path_radius around the map's centre, heading along the path;
+    scan s is a subsample of the map points within max_range (horizontally) of its position, between min_points and
+    max_points of them (ragged), plus `noise` m of Gaussian noise, in the vehicle's body frame: T_gt[s] @ scan lies on
+    the map.  T_init[s] = T_gt[s] @ dT with dT of the size of icp_pk01.yaml's initial offset (0.15 / 0.12 / 0.13 m,
+    0.015 / 1.31 / 2.17 deg), each component scaled by a seeded U[-1, 1]."""
+    _, tgt = make_parking(n_map=n_map, seed=43)
+    rng = np.random.default_rng(seed)
+    d = math.pi / 180.0
+    size = np.array([0.15, 0.12, 0.13, 0.015 * d, 1.31 * d, 2.17 * d])
+    mx, my = tgt[:, 0].astype(np.float64), tgt[:, 1].astype(np.float64)
+    scans, T_gt, T_init = [], [], []
+    for s in range(n_scans):
+        th = 2.0 * math.pi * s / n_scans
+        T = pose6d_to_matrix(path_radius * math.cos(th), path_radius * math.sin(th), 0.0, 0.0, 0.0, th + math.pi / 2)
+        cand = np.nonzero((mx - T[0, 3]) ** 2 + (my - T[1, 3]) ** 2 < max_range * max_range)[0]
+        k = min(int(rng.integers(min_points, max_points + 1)), cand.size)
+        pick = np.sort(rng.choice(cand, size=k, replace=False))
+        world = tgt[pick].astype(np.float64) + rng.normal(0, noise, (k, 3))
+        scans.append(np.ascontiguousarray(((world - T[:3, 3]) @ T[:3, :3]).astype(np.float32)))
+        dT = pose6d_to_matrix(*(size * rng.uniform(-1.0, 1.0, 6)))
+        T_gt.append(T)
+        T_init.append(T @ dT)
+    return scans, tgt, np.array(T_gt), np.array(T_init)
 
 
 def trial_poses(n, seed=45, max_trans=1.0, max_rot_deg=3.0):

@@ -221,6 +221,21 @@ int dcreg_icp_fetch(dcreg_ctx* ctx, double T_out[16], int* n_iterations, int* co
 int dcreg_icp_run_batch(dcreg_ctx* ctx, const dcreg_icp_params* params, int n_trials, const double* T_init,
                         double* T_out, int* n_iterations, int* converged, int* status, dcreg_iter_log* log,
                         int log_cap);
+/* Many DIFFERENT source scans registered against the context's target (e.g. every frame of a recorded sequence
+ * against one prior map, each from its own initial guess), side by side: scan s = points
+ * [scan_offsets[s], scan_offsets[s+1]) of xyz (`stride` floats per point), trial = scan.  T_init / T_out /
+ * n_iterations / converged / status / log as in dcreg_icp_run_batch (log trial-major, n_scans x log_cap).
+ * fitness of scan s is over its own point count.  The context's source (dcreg_set_source) is not replaced.
+ * Every scan runs the kernels a dcreg_icp_run of that scan alone from the same T_init runs (the scan is sorted by
+ * target cell under its own T_init and uses its own lever arm): counts, masks and iteration counts are identical,
+ * poses equal up to the grouping of the FP64 sums (1e-8 in the tests); a one-scan call IS a dcreg_icp_run, bit for bit,
+ * and a call is reproducible bit for bit.  n_scans in [1, 65535]; scan_offsets[0] = 0 and strictly increasing (no empty
+ * scan); at most 0x1fffffff points in all.  Needs the dense grid; not available on a sharded context (distribute the
+ * scans over ranks instead). */
+int dcreg_icp_run_scans(dcreg_ctx* ctx, const dcreg_icp_params* params, int n_scans,
+                        const float* xyz, int stride, const int64_t* scan_offsets,
+                        const double* T_init, double* T_out, int* n_iterations, int* converged, int* status,
+                        dcreg_iter_log* log, int log_cap);
 /* Same loop, but correspondences are supplied by the caller each iteration through a callback
  * (host kd-tree mode, "PR1"): planes are 4*n doubles (nx,ny,nz,d), all-zero = none. */
 typedef int (*dcreg_plane_callback)(void* user, const double T[16], double* planes4,
@@ -232,6 +247,10 @@ int dcreg_icp_run_host_planes(dcreg_ctx* ctx, const dcreg_icp_params* params,
 /* Post-loop covariance (icp_test_runner.cpp:2014-2037): inverse of the last H with the 1e-9
  * eigenvalue floor, or 1e6*I when not converged.  cov: 36 doubles. */
 int dcreg_last_covariance(dcreg_ctx* ctx, double cov[36]);
+/* The same for each of the first n_trials trials of the last run (dcreg_icp_run: 1; dcreg_icp_run_batch /
+ * dcreg_icp_run_scans: their trial count): cov = n_trials x 36 doubles, trial-major.  Trial 0 equals
+ * dcreg_last_covariance bit for bit.  n_trials above the last run's trial count is refused. */
+int dcreg_last_covariances(dcreg_ctx* ctx, int n_trials, double* cov);
 
 /* Post-run point-to-point metrics on the device.  Replaces calculatePointToPointError
  * (DCReg/include/utils.hpp:538-589; callers icp_test_runner.cpp:506-510 and :1463-1470): aligned = fl32(T * source);
