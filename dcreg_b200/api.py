@@ -87,7 +87,7 @@ EXPORTS = [
     "dcreg_stream", "dcreg_set_source", "dcreg_set_target", "dcreg_find_planes",
     "dcreg_reduce_normal_equations", "dcreg_reduce_normal_equations_f64plane",
     "dcreg_reduce_normal_equations_host", "dcreg_analyze_and_solve", "dcreg_solve_pcg", "dcreg_icp_run",
-    "dcreg_icp_run_batch", "dcreg_icp_run_scans", "dcreg_icp_enqueue", "dcreg_icp_fetch", "dcreg_icp_run_host_planes", "dcreg_comm_mode", "dcreg_last_covariance", "dcreg_last_covariances", "dcreg_point_to_point_metrics", "dcreg_comm_unique_id", "dcreg_comm_init",
+    "dcreg_icp_run_batch", "dcreg_icp_run_scans", "dcreg_icp_enqueue", "dcreg_icp_fetch", "dcreg_icp_run_host_planes", "dcreg_comm_mode", "dcreg_last_covariance", "dcreg_last_covariances", "dcreg_point_to_point_metrics", "dcreg_point_to_point_metrics_batch", "dcreg_comm_unique_id", "dcreg_comm_init",
     "dcreg_comm_destroy", "dcreg_set_global_source_count", "dcreg_launch_count", "dcreg_device_source",
     "dcreg_device_planes_f64", "dcreg_device_planes_f32", "dcreg_freeze_planes_f32", "dcreg_time_reduce", "dcreg_time_iteration", "dcreg_iteration_counters", "dcreg_iteration_timeline",
 ]
@@ -132,6 +132,7 @@ def load_library():
     lib.dcreg_last_covariance.argtypes = [vp, dp]
     lib.dcreg_last_covariances.argtypes = [vp, ci, dp]
     lib.dcreg_point_to_point_metrics.argtypes = [vp, dp, C.c_double, dp]
+    lib.dcreg_point_to_point_metrics_batch.argtypes = [vp, ci, dp, C.c_double, dp]
     lib.dcreg_comm_unique_id.argtypes = [vp, C.POINTER(C.c_uint8)]
     lib.dcreg_comm_init.argtypes = [vp, C.POINTER(C.c_uint8), ci, ci]
     lib.dcreg_comm_destroy.argtypes = [vp]
@@ -460,6 +461,16 @@ class Context:
         out = np.empty(4)
         self._check(self.lib.dcreg_point_to_point_metrics(self._h, _dptr(T), float(error_threshold), _dptr(out)))
         return {"rmse": out[0], "fitness": out[1], "chamfer": out[2], "n_valid": int(out[3])}
+
+    def point_to_point_metrics_batch(self, T, error_threshold: float):
+        """point_to_point_metrics for many poses in one call: T (n, 4, 4).  Returns dict of arrays rmse, fitness,
+        chamfer (float64) and n_valid (int64), each (n,); row i equals point_to_point_metrics(T[i]) bit for bit."""
+        T = np.ascontiguousarray(T, dtype=np.float64).reshape(-1, 4, 4)
+        out = np.empty((T.shape[0], 4))
+        self._check(self.lib.dcreg_point_to_point_metrics_batch(self._h, T.shape[0], _dptr(T), float(error_threshold),
+                                                                _dptr(out)))
+        return {"rmse": out[:, 0].copy(), "fitness": out[:, 1].copy(), "chamfer": out[:, 2].copy(),
+                "n_valid": out[:, 3].astype(np.int64)}
 
     # -- multi-GPU --
     def comm_unique_id(self) -> bytes:

@@ -10,7 +10,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libdcreg_b200.so")
 SOURCES = ["dcreg_b200.cu"]
-HEADERS = ["corr.cuh", "k1_reduce.cuh", "k1_stream.cuh", "k2_solve.cuh", "k2_fast.cuh", "peer_reduce.cuh", "loop_plan.hpp", "small_la.cuh",
+HEADERS = ["corr.cuh", "k1_reduce.cuh", "k1_stream.cuh", "k2_solve.cuh", "k2_fast.cuh", "peer_reduce.cuh", "loop_plan.hpp", "p2p_bound.hpp", "small_la.cuh",
            "../../include/dcreg_b200.h"]
 
 NVCC_FLAGS = [

@@ -824,6 +824,147 @@ __global__ void transform_points_kernel(const float4* __restrict__ in, long long
                          (float)(T[8] * px + T[9] * py + T[10] * pz + T[11]), p.w);
 }
 
+// ---- point-to-point metrics for many poses (dcreg_point_to_point_metrics_batch) ---------------------------------
+// Pose records: 16 doubles each, [0..11] the top three rows of T, [12] margin, [13] shrink (p2p_bound.hpp).
+constexpr int kPoseRec = 16;
+
+// fl32(T p): the expression of nn1_metrics_kernel / transform_points_kernel, so every point lands on the same float
+__device__ __forceinline__ float3 posed_point(const double* __restrict__ T, const float4 p) {
+    const double px = p.x, py = p.y, pz = p.z;
+    return make_float3((float)(T[0] * px + T[1] * py + T[2] * pz + T[3]), (float)(T[4] * px + T[5] * py + T[6] * pz + T[7]),
+                       (float)(T[8] * px + T[9] * py + T[10] * pz + T[11]));
+}
+
+// cell coordinate of an FP64 position, clamped so a far query cannot overflow int (a clamped cell is nearer to the
+// grid box than the true one, so the ring bounds below stay lower bounds)
+__device__ __forceinline__ int cell_coord_clamped(double v, double inv_cell) {
+    return (int)fmin(fmax(floor(v * inv_cell), -1073741824.0), 1073741824.0);
+}
+
+__device__ __forceinline__ float posed_scan_range(const Grid& g, const double* __restrict__ T, int s, int e, float yx,
+                                                  float yy, float yz, float best) {
+#pragma unroll 1
+    for (int j = s; j < e; ++j) {
+        const float3 a = posed_point(T, __ldg(&g.pts[j]));
+        best = fminf(best, dist2(yx, yy, yz, make_float4(a.x, a.y, a.z, 0.f)));
+    }
+    return best;
+}
+
+// Smallest float d2(y, fl32(T p)) over the source points p of a dense grid built in the source's own frame: the
+// value nn1_search returns for y over a grid built on the aligned copy.  Same ring walk around q' = R^T (y - t);
+// a ring is skipped by the bound (*) of p2p_bound.hpp, which keeps the minimum exact.
+__device__ __forceinline__ float nn1_search_posed(const Grid& g, const double* __restrict__ T, float yx, float yy, float yz) {
+    const double vx = (double)yx - T[3], vy = (double)yy - T[7], vz = (double)yz - T[11];
+    const double qx = T[0] * vx + T[4] * vy + T[8] * vz, qy = T[1] * vx + T[5] * vy + T[9] * vz, qz = T[2] * vx + T[6] * vy + T[10] * vz;
+    const double margin = T[12], shrink = T[13];
+    const double cell = 1.0 / g.inv_cell;
+    const int lx = cell_coord_clamped(qx, g.inv_cell) - g.ox, ly = cell_coord_clamped(qy, g.inv_cell) - g.oy,
+              lz = cell_coord_clamped(qz, g.inv_cell) - g.oz;
+    const int ox = lx < 0 ? -lx : (lx >= g.nx ? lx - g.nx + 1 : 0);
+    const int oy = ly < 0 ? -ly : (ly >= g.ny ? ly - g.ny + 1 : 0);
+    const int oz = lz < 0 ? -lz : (lz >= g.nz ? lz - g.nz + 1 : 0);
+    const int r0 = max(ox, max(oy, oz));
+    const int r1 = max(max(lx, g.nx - 1 - lx), max(max(ly, g.ny - 1 - ly), max(lz, g.nz - 1 - lz)));
+    float best = 3.0e38f;
+#pragma unroll 1
+    for (int r = r0; r <= r1; ++r) {
+        if (r > 0) {
+            const double l = (double)(r - 1) * cell * 0.99999 - margin;
+            if (l > 0.0 && l * l * shrink > (double)best) break;
+        }
+        const int z0 = max(-r, -lz), z1 = min(r, g.nz - 1 - lz);
+        const int y0 = max(-r, -ly), y1 = min(r, g.ny - 1 - ly);
+#pragma unroll 1
+        for (int dz = z0; dz <= z1; ++dz) {
+#pragma unroll 1
+            for (int dy = y0; dy <= y1; ++dy) {
+                const int* rowp = g.cell_start + (size_t)((lz + dz) * g.ny + (ly + dy)) * g.nx;
+                const bool shell = (dz == -r) || (dz == r) || (dy == -r) || (dy == r);
+                if (shell) {                                         // whole x-span of the ring, one contiguous range
+                    const int xa = max(lx - r, 0), xb = min(lx + r, g.nx - 1);
+                    if (xa > xb) continue;
+                    best = posed_scan_range(g, T, __ldg(rowp + xa), __ldg(rowp + xb + 1), yx, yy, yz, best);
+                } else {                                             // interior row: only the two end cells dx = +-r
+                    for (int sgn = -1; sgn <= 1; sgn += 2) {
+                        const int xx = lx + sgn * r;
+                        if (xx < 0 || xx >= g.nx) continue;
+                        best = posed_scan_range(g, T, __ldg(rowp + xx), __ldg(rowp + xx + 1), yx, yy, yz, best);
+                    }
+                }
+            }
+        }
+    }
+    return best;
+}
+
+// Forward pass, blockIdx.y = pose: nn1_metrics_kernel's decomposition and per-block partials for each pose.
+__global__ void nn1_metrics_poses_kernel(const float4* __restrict__ q, long long n, const double* __restrict__ poses, Grid g,
+                                         double threshold, double* __restrict__ partials) {
+    __shared__ double sh[3][8];
+    const double* T = poses + (size_t)blockIdx.y * kPoseRec;
+    double sd = 0.0, ssq = 0.0, cnt = 0.0;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const float3 a = posed_point(T, __ldg(&q[i]));
+        const float d2 = nn1_search(g, a.x, a.y, a.z);
+        const double dist = sqrt((double)d2);
+        sd += dist;
+        if (dist < threshold) { ssq += (double)d2; cnt += 1.0; }
+    }
+    for (int off = 16; off > 0; off >>= 1) {
+        sd += __shfl_down_sync(0xffffffffu, sd, off);
+        ssq += __shfl_down_sync(0xffffffffu, ssq, off);
+        cnt += __shfl_down_sync(0xffffffffu, cnt, off);
+    }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (lane == 0) { sh[0][warp] = sd; sh[1][warp] = ssq; sh[2][warp] = cnt; }
+    __syncthreads();
+    if (threadIdx.x < 3) {
+        double s = 0.0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += sh[threadIdx.x][w];
+        partials[((size_t)blockIdx.y * gridDim.x + blockIdx.x) * 3 + threadIdx.x] = s;
+    }
+}
+
+// Backward (Chamfer) pass, blockIdx.y = pose: target point -> nearest aligned source point through the source-frame
+// grid; per-block sum of distances in nn1_metrics_kernel's order.
+__global__ void nn1_chamfer_poses_kernel(const float4* __restrict__ tgt, long long m, const double* __restrict__ poses,
+                                         Grid gs, double* __restrict__ partials) {
+    __shared__ double sh[8];
+    const double* T = poses + (size_t)blockIdx.y * kPoseRec;
+    double sd = 0.0;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += (long long)gridDim.x * blockDim.x) {
+        const float4 y = __ldg(&tgt[i]);
+        sd += sqrt((double)nn1_search_posed(gs, T, y.x, y.y, y.z));
+    }
+    for (int off = 16; off > 0; off >>= 1) sd += __shfl_down_sync(0xffffffffu, sd, off);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (lane == 0) sh[warp] = sd;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double s = 0.0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += sh[w];
+        partials[(size_t)blockIdx.y * gridDim.x + blockIdx.x] = s;
+    }
+}
+
+// One thread per pose: the host sums of dcreg_point_to_point_metrics (block order 0..grid-1), then
+// out = { sqrt(sum_sq / n), count / n, (sum_f / n + sum_b / m) / 2, count }.
+__global__ void p2p_finish_kernel(const double* __restrict__ pf, int gridf, const double* __restrict__ pb, int gridb,
+                                  int n_poses, long long n, long long m, double* __restrict__ out) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_poses) return;
+    double sum_fwd = 0, sum_sq = 0, valid = 0, sum_bwd = 0;
+    const double* f = pf + (size_t)k * gridf * 3;
+    for (int b = 0; b < gridf; ++b) { sum_fwd += f[3 * b]; sum_sq += f[3 * b + 1]; valid += f[3 * b + 2]; }
+    const double* bb = pb + (size_t)k * gridb;
+    for (int b = 0; b < gridb; ++b) sum_bwd += bb[b];
+    out[4 * k + 0] = sqrt(sum_sq / (double)n);
+    out[4 * k + 1] = valid / (double)n;
+    out[4 * k + 2] = 0.5 * (sum_fwd / (double)n + sum_bwd / (double)m);
+    out[4 * k + 3] = valid;
+}
+
 // Plane through the 5 neighbours: least squares of [nb] x = -1, n = x/|x|, d = 1/|x|, gates
 // |x| >= min_norm and max_j (n.nb_j + d)^2 < thickness^2 (icp_test_runner.cpp:1727-1773).
 // Returns true and (n, d) when a valid plane exists.

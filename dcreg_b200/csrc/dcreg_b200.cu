@@ -32,6 +32,7 @@
 #include "k1_stream.cuh"
 #include "k2_solve.cuh"
 #include "loop_plan.hpp"
+#include "p2p_bound.hpp"
 #include "peer_reduce.cuh"
 
 using k2::IcpState;
@@ -776,6 +777,10 @@ struct dcreg_ctx {
     int* d_pt_cell = nullptr; long long pt_cell_cap = 0;
     int* d_tile_sums = nullptr; long long tile_sums_cap = 0;
     double cell_size = 0.0;
+    // dcreg_point_to_point_metrics_batch: grid over the source in its own frame (cell_size), dropped by set_source /
+    // set_target; pose records + partial sums + results of one chunk of poses
+    corr::Grid src_grid{}; bool has_src_grid = false;
+    double* d_p2p = nullptr; long long p2p_cap = 0;
 
     double4* d_planes64 = nullptr; float4* d_planes32 = nullptr; long long planes_cap = 0;
 
@@ -1104,7 +1109,8 @@ int dcreg_destroy(dcreg_ctx* ctx) {
                     ctx->grid.hcount, ctx->d_src_sorted, ctx->d_cell_tmp, ctx->d_pt_cell, ctx->d_tile_sums,
                     ctx->grid.pts, ctx->grid.pos_of, ctx->d_planes64, ctx->d_planes32, ctx->d_partials, ctx->d_counter, ctx->d_acc,
                     ctx->d_state, ctx->d_log, ctx->d_small, ctx->d_analysis, ctx->d_flush, ctx->d_nn, ctx->d_plane_cache, ctx->d_fit_state, ctx->d_iter_stats, ctx->d_src_radius, ctx->d_plane_key, ctx->d_k2_scratch,
-                    ctx->d_cov, ctx->d_scan, ctx->d_scan_sorted, ctx->d_scan_keys, ctx->d_scan_slots, ctx->d_scan_sort_tmp, ctx->d_scan_off, ctx->d_scan_radius};
+                    ctx->d_cov, ctx->d_scan, ctx->d_scan_sorted, ctx->d_scan_keys, ctx->d_scan_slots, ctx->d_scan_sort_tmp, ctx->d_scan_off, ctx->d_scan_radius,
+                    ctx->src_grid.keys, ctx->src_grid.cell_start, ctx->src_grid.hstart, ctx->src_grid.hcount, ctx->src_grid.pts, ctx->src_grid.pos_of, ctx->d_p2p};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
@@ -1120,10 +1126,14 @@ void* dcreg_device_source(dcreg_ctx* ctx) { return ctx ? ctx->d_src : nullptr; }
 void* dcreg_device_planes_f64(dcreg_ctx* ctx) { return ctx ? ctx->d_planes64 : nullptr; }
 void* dcreg_device_planes_f32(dcreg_ctx* ctx) { return ctx ? ctx->d_planes32 : nullptr; }
 
+static void free_grid(corr::Grid* g);
+
 int dcreg_set_source(dcreg_ctx* ctx, const float* xyz, int64_t n, int stride) {
     if (!ctx) return DCREG_BAD_ARG;
     if (!xyz || n <= 0 || stride < 3) { ctx->err = "dcreg_set_source: empty cloud or stride < 3"; return DCREG_BAD_ARG; }
     CK(cudaSetDevice(ctx->device));
+    free_grid(&ctx->src_grid);
+    ctx->has_src_grid = false;
     if (ctx->n_src_cap < n) {
         if (ctx->d_src) cudaFree(ctx->d_src);
         ctx->d_src = nullptr; ctx->n_src_cap = 0;
@@ -1183,7 +1193,7 @@ static int build_grid(dcreg_ctx* ctx, const float4* d_pts, long long m, double c
     CK(cudaStreamSynchronize(ctx->stream));
     for (int k = 0; k < 3; ++k)
         if (hb[k] < -(1 << 19) || hb[3 + k] > (1 << 19)) {
-            cudaFree(g.pts);
+            cudaFree(g.pts); cudaFree(g.pos_of);
             ctx->err = "grid build: coordinates / cell_size exceed the +-2^19 cell range (NaN or huge coordinates?)";
             return DCREG_BAD_ARG;
         }
@@ -1251,6 +1261,8 @@ int dcreg_set_target(dcreg_ctx* ctx, const float* xyz, int64_t m, int stride, do
     ctx->d_tgt = nullptr;
     free_grid(&ctx->grid);
     ctx->has_grid = false;
+    free_grid(&ctx->src_grid);   // built with the target's cell size
+    ctx->has_src_grid = false;
     CK(cudaMalloc(&ctx->d_tgt, (size_t)m * sizeof(float4)));
     ctx->n_tgt = m;
     int rc = upload_points(ctx, xyz, m, stride, ctx->d_tgt, nullptr);
@@ -1309,6 +1321,84 @@ int dcreg_point_to_point_metrics(dcreg_ctx* ctx, const double T[16], double erro
     out[1] = valid / (double)n;
     out[2] = 0.5 * (sum_fwd / (double)n + sum_bwd / (double)m);
     out[3] = valid;
+    return DCREG_OK;
+}
+
+// upper bound of |p| over the points of a dense grid, from its cell box
+static double grid_box_radius(const corr::Grid& g) {
+    const double cell = 1.0 / g.inv_cell;
+    const int lo[3] = {g.ox, g.oy, g.oz}, len[3] = {g.nx, g.ny, g.nz};
+    double s = 0.0;
+    for (int k = 0; k < 3; ++k) {
+        const double a = fmax(fabs((double)lo[k]), fabs((double)lo[k] + len[k])) * cell;
+        s += a * a;
+    }
+    return sqrt(s) * (1.0 + 1e-9);
+}
+
+// Partial sums of one chunk of poses stay below this many doubles (32 MB); the chunk size does not change results.
+constexpr long long kP2pChunkDoubles = 1LL << 22;
+
+// dcreg_point_to_point_metrics for many poses: the forward pass is nn1_metrics_kernel's decomposition per pose
+// (blockIdx.y), the backward pass searches one cached grid over the source in its own frame instead of building a
+// grid over every aligned copy (nn1_search_posed, exact by the bound of p2p_bound.hpp), and p2p_finish_kernel forms
+// each pose's metrics from its partials in the host's summation order.  No device allocation once the buffers have grown,
+// one synchronisation per call.
+int dcreg_point_to_point_metrics_batch(dcreg_ctx* ctx, int n_poses, const double* T, double error_threshold, double* out) {
+    if (!ctx) return DCREG_BAD_ARG;
+    if (n_poses < 1) { ctx->err = "p2p metrics batch: n_poses < 1"; return DCREG_BAD_ARG; }
+    if (!T || !out) { ctx->err = "p2p metrics batch: null pointer"; return DCREG_BAD_ARG; }
+    if (!ctx->d_src || !ctx->has_grid || !ctx->d_tgt) { ctx->err = "p2p metrics batch: set source and target first"; return DCREG_BAD_ARG; }
+    if (!ctx->grid.dense) { ctx->err = "p2p metrics batch needs the dense grid (target bounding box too large for this cell size)"; return DCREG_BAD_ARG; }
+    CK(cudaSetDevice(ctx->device));
+    const long long n = ctx->n_src, m = ctx->n_tgt;
+    if (!ctx->has_src_grid) {
+        if (n > 0x7fffffffLL) { ctx->err = "p2p metrics batch: too many source points"; return DCREG_BAD_ARG; }
+        corr::Grid g{};
+        int rc = build_grid(ctx, ctx->d_src, n, ctx->cell_size, &g, nullptr);
+        if (rc) return rc;
+        if (!g.dense) {
+            free_grid(&g);
+            ctx->err = "p2p metrics batch needs a dense grid over the source (source bounding box too large for this cell size)";
+            return DCREG_BAD_ARG;
+        }
+        ctx->src_grid = g; ctx->has_src_grid = true;
+    }
+    const corr::Grid& gs = ctx->src_grid;
+    const int gridf = stream_grid(ctx, n, 8), gridb = stream_grid(ctx, m, 8);
+    const long long part = 3LL * gridf + gridb;                  // partial sums per pose
+    long long chunk = std::min<long long>({(long long)n_poses, 65535LL, std::max<long long>(1, kP2pChunkDoubles / part)});
+    if (const char* s = getenv("DCREG_P2P_CHUNK")) {             // smaller chunks, for tests of the chunking
+        const long long c = atoll(s);
+        if (c >= 1 && c < chunk) chunk = c;
+    }
+    // layout of d_p2p: pose records [n_poses][kPoseRec] | results [n_poses][4] | forward partials | backward partials
+    int rc = ensure_buffer(ctx, &ctx->d_p2p, &ctx->p2p_cap, (long long)n_poses * (corr::kPoseRec + 4) + chunk * part);
+    if (rc) return rc;
+    double* d_rec = ctx->d_p2p;
+    double* d_out = d_rec + (size_t)n_poses * corr::kPoseRec;
+    double* d_pf = d_out + (size_t)n_poses * 4;
+    double* d_pb = d_pf + (size_t)chunk * 3 * gridf;
+    const double pmax = grid_box_radius(gs), ymax = grid_box_radius(ctx->grid);
+    std::vector<double> rec((size_t)n_poses * corr::kPoseRec, 0.0);
+    for (int k = 0; k < n_poses; ++k) {
+        double* r = &rec[(size_t)k * corr::kPoseRec];
+        memcpy(r, T + (size_t)k * 16, 12 * sizeof(double));
+        const p2p_bound::Bound b = p2p_bound::backward_bound(T + (size_t)k * 16, pmax, ymax);
+        r[12] = b.margin; r[13] = b.shrink;
+    }
+    CK(cudaMemcpyAsync(d_rec, rec.data(), rec.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    for (long long c0 = 0; c0 < n_poses; c0 += chunk) {
+        const int cnt = (int)std::min<long long>(chunk, n_poses - c0);
+        const double* r = d_rec + (size_t)c0 * corr::kPoseRec;
+        corr::nn1_metrics_poses_kernel<<<dim3(gridf, cnt), kBlock, 0, ctx->stream>>>(ctx->d_src, n, r, ctx->grid, error_threshold, d_pf);
+        corr::nn1_chamfer_poses_kernel<<<dim3(gridb, cnt), kBlock, 0, ctx->stream>>>(ctx->d_tgt, m, r, gs, d_pb);
+        corr::p2p_finish_kernel<<<(cnt + 127) / 128, 128, 0, ctx->stream>>>(d_pf, gridf, d_pb, gridb, cnt, n, m, d_out + (size_t)c0 * 4);
+        ctx->launches += 3;
+        CK(cudaGetLastError());
+    }
+    CK(cudaMemcpyAsync(out, d_out, (size_t)n_poses * 4 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
     return DCREG_OK;
 }
 

@@ -17,7 +17,8 @@
 //
 // Extension (not in the reference, which has no RNG - SURVEY.md §6 C5): an optional `monte_carlo:` block runs a seeded
 // perturbation study of every listed method through dcreg_icp_run_batch (all trials advance side by side on the GPU) and
-// writes monte_carlo_<method>.csv + monte_carlo_summary.txt.  Absent block = the reference's behaviour, unchanged.
+// writes monte_carlo_<method>.csv (ending in the point-to-point metrics of every trial's final pose, one batched
+// dcreg_point_to_point_metrics_batch call per method) + monte_carlo_summary.txt.  Absent block = the reference's behaviour, unchanged.
 #include <algorithm>
 #include <chrono>
 #include <cmath>
@@ -291,6 +292,15 @@ private:
         }
     }
 
+    // dcreg_point_to_point_metrics for every pose of T (n x 16) in one call: out = n x {rmse, fitness, chamfer, n_valid},
+    // zeros when the call fails (as p2p leaves them)
+    void p2pBatch(const std::vector<double>& T, std::vector<double>& out) {
+        const int n = (int)(T.size() / 16);
+        out.assign((size_t)n * 4, 0.0);
+        if (n > 0 && !check(dcreg_point_to_point_metrics_batch(ctx_, n, T.data(), config_.error_threshold, out.data()), "point_to_point_metrics_batch"))
+            out.assign((size_t)n * 4, 0.0);
+    }
+
     static bool isSo3Method(const std::string& name) {
         static const char* so3_names[] = {"Ours", "NONE", "ME-SR", "FCN-SR", "ME-TSVD", "ME-TReg"};
         return std::find_if(std::begin(so3_names), std::end(so3_names), [&](const char* s) { return name == s; }) != std::end(so3_names);
@@ -338,7 +348,10 @@ private:
             std::ofstream f(config_.output_folder + "monte_carlo_" + kv.first + ".csv");
             f << "Trial,Init_x,Init_y,Init_z,Init_roll_deg,Init_pitch_deg,Init_yaw_deg,Converged,Iterations,Status,Trans_Error_m,Rot_Error_deg";
             for (int k = 0; k < 12; ++k) f << ",T" << k / 4 << k % 4;
+            f << ",P2P_RMSE,P2P_Fitness,Chamfer_Distance";
             f << "\n" << std::setprecision(17);
+            std::vector<double> p2p_out;
+            p2pBatch(T1, p2p_out);
             std::vector<double> te, re;
             long long it_sum = 0; int n_conv = 0, n_fail = 0;
             for (int i = 0; i < n; ++i) {
@@ -347,6 +360,7 @@ private:
                 f << i << ',' << init[i].x << ',' << init[i].y << ',' << init[i].z << ',' << rad2deg(init[i].roll) << ',' << rad2deg(init[i].pitch) << ','
                   << rad2deg(init[i].yaw) << ',' << conv[i] << ',' << iters[i] << ',' << status[i] << ',' << e.translation_error << ',' << e.rotation_error;
                 for (int k = 0; k < 12; ++k) f << ',' << Tf.m[k];
+                f << ',' << p2p_out[(size_t)i * 4] << ',' << p2p_out[(size_t)i * 4 + 1] << ',' << p2p_out[(size_t)i * 4 + 2];
                 f << "\n";
                 if (status[i] != DCREG_OK) { ++n_fail; continue; }
                 te.push_back(e.translation_error); re.push_back(e.rotation_error);
@@ -712,14 +726,18 @@ private:
             for (int i = 0; i < 6; ++i) ic << "Degenerate_" << i << ",";
             ic << "Is_Degenerate\n";
             for (const auto& kv : detailed_results_)
-                for (size_t run = 0; run < kv.second.size(); ++run)
-                    for (size_t it = 0; it < kv.second[run].iteration_data.size(); ++it) {
-                        const IterData& d = kv.second[run].iteration_data[it];
+                for (size_t run = 0; run < kv.second.size(); ++run) {
+                    // the reference evaluates every row's pose (icp_test_runner.cpp:1460-1468); one batched call per run
+                    const std::vector<IterData>& iters = kv.second[run].iteration_data;
+                    std::vector<double> poses(iters.size() * 16), p2p_out;
+                    for (size_t it = 0; it < iters.size(); ++it) std::memcpy(&poses[it * 16], iters[it].g.T, 16 * sizeof(double));
+                    p2pBatch(poses, p2p_out);
+                    for (size_t it = 0; it < iters.size(); ++it) {
+                        const IterData& d = iters[it];
                         Mat4 Ti; std::memcpy(Ti.m, d.g.T, sizeof(Ti.m));
                         const PoseError e = calculatePoseError(config_.gt_matrix, Ti);
                         const double trans_error = e.rotation_error, rot_error = e.translation_error;   // sic (icp_test_runner.cpp:1457-1458)
-                        double p2p_rmse = 0, p2p_fit = 0, chamfer = 0; int corr = 0;
-                        p2p(Ti, p2p_rmse, p2p_fit, chamfer, corr);
+                        const double p2p_rmse = p2p_out[it * 4], chamfer = p2p_out[it * 4 + 2];
                         ic << kv.first << "," << run << "," << it << "," << d.g.rmse << "," << d.g.fitness << "," << d.iter_time_ms << ","
                            << trans_error << "," << rot_error << "," << p2p_rmse << "," << chamfer << ",";
                         for (int i = 0; i < 6; ++i) ic << d.g.dx[i] << ",";
@@ -731,6 +749,7 @@ private:
                         for (int i = 0; i < 6; ++i) ic << (a.degenerate_mask[i] ? 1 : 0) << ",";
                         ic << (a.is_degenerate ? 1 : 0) << "\n";
                     }
+                }
             std::cout << "Iteration details with dx saved to: " << config_.output_folder + "iteration_details_with_dx.csv" << std::endl;
         }
     }

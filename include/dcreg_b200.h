@@ -258,6 +258,15 @@ int dcreg_last_covariances(dcreg_ctx* ctx, int n_trials, double* cov);
  * number of source points within the threshold }.  Needs dcreg_set_source + dcreg_set_target. */
 int dcreg_point_to_point_metrics(dcreg_ctx* ctx, const double T[16], double error_threshold, double out[4]);
 
+/* dcreg_point_to_point_metrics for n_poses poses at once: T = n_poses row-major 4x4, out = n_poses x 4
+ * {rmse, fitness, chamfer, n_valid}, pose-major.  Row i equals dcreg_point_to_point_metrics(ctx, T + 16 i, ...) bit
+ * for bit.  Same preconditions (source + target set, dense target grid); n_poses >= 1.  The Chamfer half searches a
+ * grid over the source in its own frame (built on first use, cell size of the target grid, kept until the next
+ * dcreg_set_source / dcreg_set_target), so the source's bounding box must also fit a dense grid.  One host
+ * synchronisation per call. */
+int dcreg_point_to_point_metrics_batch(dcreg_ctx* ctx, int n_poses, const double* T, double error_threshold,
+                                       double* out);
+
 /* ---- multi-GPU: point-block sharding (SURVEY.md §8e) ---------------------------------------
  * Each rank holds a contiguous block of source slots; the 27+5 accumulators are summed over ranks
  * once per iteration (inside the reducing kernel over peer memory, see dcreg_comm_mode; one
